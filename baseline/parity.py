@@ -18,10 +18,14 @@ positions).  So the check is:
 
 ``report["exact"]`` is True when no position diverged; ``report["ok"]`` when every divergence is a near-tie
 (both candidates within ``tol_ulps`` of the reference's top logit).
+
+The reference is not part of this repository, so the GPU tests judge against records of its runs on a B200
+(``record_reference`` / ``compare_ids_to_record``, written by ``tests/golden/gen_golden_gpu_parity.py``).
 """
 from __future__ import annotations
 
 import contextlib
+import hashlib
 import io
 import random
 from typing import Callable, List, Optional, Sequence
@@ -145,6 +149,15 @@ def reference_self_consistency(ref_model, ref_ids: Sequence[int], n_prompt: int)
             "how": "reference lookahead ids vs the reference model's own teacher-forced causal forward (argmax per position)"}
 
 
+def weights_digest(model) -> str:
+    """sha256 over the parameter names and bytes: a record of the reference holds only for the weights it ran on."""
+    h = hashlib.sha256()
+    for name, p in sorted(model.named_parameters()):
+        h.update(name.encode())
+        h.update(p.detach().contiguous().view(torch.uint8).cpu().numpy().tobytes())
+    return h.hexdigest()
+
+
 def _mant_bits(model) -> int:
     """Explicit mantissa bits of the model dtype: the unit in which a logit 'tie' is measured (bf16 7, fp16 10)."""
     return {torch.bfloat16: 7, torch.float16: 10}.get(next(model.parameters()).dtype, 23)
@@ -167,8 +180,46 @@ def compare_ids(our_generate: Callable[[List[int], int], List[int]], ref_ids: Se
     The tolerance is max(tol_ulps, the reference's own self-inconsistency on this run): a divergence no wider than
     the distance at which the reference disagrees with itself cannot be told apart from a tie."""
     ref_ids = list(ref_ids)
+    self_rep = reference_self_consistency(ref_model, ref_ids, n_prompt) if self_check and len(ref_ids) - n_prompt >= 1 else None
+    return _compare_on_logits(our_generate, ref_ids, n_prompt, lambda prefix: reference_next_logits(ref_model, prefix),
+                              _mant_bits(ref_model), self_rep, tol_ulps, max_divergences)
+
+
+def record_reference(ref_model, ref_ids: Sequence[int], n_prompt: int, top_k: int = 32) -> dict:
+    """What compare_ids reads from the reference model, recorded so that the comparison can run without it: the ids,
+    the self-consistency report, the mantissa bits of the model dtype and, at every generated position i, the top
+    `top_k` of reference_next_logits(ref_ids[:i]) (values are model-dtype numbers, exact in fp32)."""
+    ref_ids = list(ref_ids)
+    top_idx, top_val = [], []
+    for i in range(n_prompt, len(ref_ids)):
+        t = torch.topk(reference_next_logits(ref_model, ref_ids[:i]), top_k)
+        top_idx.append(t.indices.tolist())
+        top_val.append(t.values.tolist())
+    return {"ids": ref_ids, "n_prompt": n_prompt, "mant_bits": _mant_bits(ref_model),
+            "self_consistency": reference_self_consistency(ref_model, ref_ids, n_prompt), "top_idx": top_idx,
+            "top_val": top_val}
+
+
+def compare_ids_to_record(our_generate: Callable[[List[int], int], List[int]], rec: dict, vocab: int,
+                          tol_ulps: float = 3.0, max_divergences: int = 64) -> dict:
+    """compare_ids against a record_reference() record.  A token outside the recorded top-k gets -inf as its logit:
+    a divergence to it is never taken for a tie."""
+    ref_ids, n_prompt = list(rec["ids"]), rec["n_prompt"]
+
+    def next_logits(prefix):
+        i = len(prefix)
+        assert list(prefix) == ref_ids[:i] and n_prompt <= i < len(ref_ids), "not a recorded prefix"
+        logits = torch.full((vocab,), -float("inf"))
+        logits[torch.tensor(rec["top_idx"][i - n_prompt])] = torch.tensor(rec["top_val"][i - n_prompt])
+        return logits
+    return _compare_on_logits(our_generate, ref_ids, n_prompt, next_logits, rec["mant_bits"], rec["self_consistency"],
+                              tol_ulps, max_divergences)
+
+
+def _compare_on_logits(our_generate, ref_ids: List[int], n_prompt: int, next_logits: Callable[[List[int]], torch.Tensor],
+                       mant_bits: int, self_rep: Optional[dict], tol_ulps: float, max_divergences: int) -> dict:
+    """The loop of compare_ids; next_logits(prefix) -> the reference model's fp32 [V] logits after that prefix."""
     total = len(ref_ids)
-    self_rep = reference_self_consistency(ref_model, ref_ids, n_prompt) if self_check and total - n_prompt >= 1 else None
     if self_rep is not None:
         tol_ulps = max(tol_ulps, self_rep["worst_below_top_ulps"])
     ours = list(our_generate(ref_ids[:n_prompt], total - n_prompt))
@@ -180,9 +231,9 @@ def compare_ids(our_generate: Callable[[List[int], int], List[int]], ref_ids: Se
         if i is None:
             length_ok = len(ours) == total
             break
-        logits = reference_next_logits(ref_model, ref_ids[:i])
+        logits = next_logits(ref_ids[:i])
         top = logits.max().item()
-        ulp = _bf16_ulp(top, _mant_bits(ref_model))
+        ulp = _bf16_ulp(top, mant_bits)
         la, lb = logits[ours[i]].item(), logits[ref_ids[i]].item()
         srt = torch.topk(logits, 2).values
         divergences.append({"index": i - n_prompt, "ours": int(ours[i]), "ref": int(ref_ids[i]),

@@ -14,7 +14,8 @@ this image, using the five small shims of SURVEY.md App. C.  Users:
   * ``bench.py``: the ``--impl reference`` arm (the unmodified reference on the host cores), the
     ``reference_cuda_eager`` leg (the same loop on the GPU: the denominator of the north star's 1.8x) and the
     ``parity`` field (token ids of our engine against the reference's on the same GPU, ``baseline/parity.py``);
-  * ``-m gpu`` parity tests (``tests/test_gpu_vs_reference.py``).
+  * ``tests/golden/gen_golden_gpu_parity.py``: the reference's GPU runs that the ``-m gpu`` parity tests
+    (``tests/test_gpu_vs_reference.py``) are judged against.
 
 Nothing in the product package may import this file.  ``/root/reference`` does not exist on the GPU box: there the
 root is ``baseline/_ref`` (``default_reference_root()``).

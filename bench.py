@@ -8,6 +8,7 @@ surface (lade.augment_all(); lade.config_lade(...); model.generate(...)) with th
 memory and the output read back to the host inside the timed region.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload 7b|13b|tiny]
+                  [--dump-outputs DIR]
 
 Extra objects on the JSON line: `roofline` (lookahead-attention kernel, HBM bound, timed live with CUDA
 events), `cpu_baseline` (the oracle port of the reference's loop on the host cores, bounded sample),
@@ -40,10 +41,17 @@ WORKLOAD_NAMES = {"7b": "Llama-2-7B-shaped random-init bf16, greedy", "13b": "Co
                   "tiny": "tiny random-init Llama (2 layers, hidden 256), greedy"}
 
 
+def _positive_int(v):
+    n = int(v)
+    if n < 1:
+        raise argparse.ArgumentTypeError(f"{v} is not >= 1")
+    return n
+
+
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=_positive_int, default=3)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="7b", choices=sorted(WORKLOADS))
@@ -64,12 +72,19 @@ def parse():
                          "rank keeps about the single-GPU row count: the lookahead capacity grows with N, not the per-rank "
                          "work); not the BASELINE config -- the line says so in config.workload")
     ap.add_argument("--ref-budget-s", type=float, default=240.0,
-                    help="--impl reference: wall-clock bound of the timed steady steps")
+                    help="--impl reference: wall-clock bound of the timed steady steps; once 3 are in, it ends the "
+                         "sample before --steps (the JSON line's `steps` says how many were timed)")
     ap.add_argument("--no-reference-cuda", action="store_true",
                     help="skip timing the unmodified reference's CUDA-eager loop (needs baseline/_ref)")
     ap.add_argument("--cuda-profiler-range", action="store_true",
                     help="cudaProfilerStart/Stop around the timed region (use with ncu --profile-from-start off)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the ids the last timed generate() returned (DIR/output_ids.npy) "
+                         "and those of the last end-to-end generate() (DIR/e2e_output_ids.npy), float64, prompt included")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm times a bounded sample of steps and has no outputs")
+    return args
 
 
 def measured_peaks():
@@ -555,12 +570,14 @@ def main():
         # its loop (a bounded sample of the workload); W untimed + K timed, the whole-workload tokens/s follows from
         # prefill + window fill (timed once) + (max_new - N + 2) steady steps.
         n_threads = usable_cores()
-        cb = reference_cpu(shape, W, N, G, P, args.max_new, n_threads, timed_steps=max(3, args.steps),
+        cb = reference_cpu(shape, W, N, G, P, args.max_new, n_threads, timed_steps=args.steps,
                            warm_steps=max(0, args.warmup), budget_s=args.ref_budget_s, weights=args.weights)
         if "unavailable" in cb:
             print(json.dumps({"impl": "reference", "unavailable": cb["unavailable"]}))
             return
-        line = {"metric": metric, "value": cb["value"], "unit": "tokens/s", "n_gpus": args.gpus, "steps": args.steps,
+        # --steps steady steps are timed unless --ref-budget-s runs out first (never below 3) or the run ends by itself
+        line = {"metric": metric, "value": cb["value"], "unit": "tokens/s", "n_gpus": args.gpus,
+                "steps": cb["steady_steps_timed"],
                 "warmup": args.warmup, "ms_per_step": round(1e3 * cb["s_per_steady_step"], 1), "higher_is_better": True,
                 "scaling": "weak", "vs_baseline": None, "dtype": "bf16", "data": "synthetic", "config": config,
                 "impl": "reference", "accepted_tokens_per_step": cb["accepted_tokens_per_step"], "cpu_baseline": cb,
@@ -710,6 +727,11 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "output_ids.npy"), np.asarray(out, dtype=np.float64))
+        np.save(os.path.join(args.dump_outputs, "e2e_output_ids.npy"), np.asarray(e2e_ids, dtype=np.float64))
     clocks = sampler.summary()
     roof = attn_roofline(eng, shape)
 

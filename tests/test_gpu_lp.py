@@ -147,7 +147,7 @@ def _full_window0(c):
     return best
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs >= 2 GPUs (run under gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs >= 2 GPUs")
 @pytest.mark.parametrize("world", [w for w in (2, 4, 8) if w <= max(torch.cuda.device_count(), 2)])
 def test_engine_lp_over_nccl_matches_single_gpu(world):
     """Real NCCL run: torchrun x `world` ranks, lade.config_lade(DIST_WORKERS=world); ids == single-GPU ids."""

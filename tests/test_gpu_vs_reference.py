@@ -1,5 +1,7 @@
-"""GPU-vs-GPU token-id parity: this repo's engine against the UNMODIFIED reference (baseline/_ref) run on the same B200
-with the same weight tensors (baseline/parity.py).
+"""GPU token-id parity: this repo's engine against the UNMODIFIED reference run on a B200 with the same weight tensors.
+The reference is not part of the repository: its runs are recorded in tests/golden/reference_gpu_parity.json.gz
+(tests/golden/gen_golden_gpu_parity.py; ids, self-consistency and the top-32 next-token logits at every position,
+baseline/parity.py) together with a digest of the weights they ran on.
 
 BASELINE.json config 1 (tiny random-init Llama, W5 N3 G3 -- with head_dim 128 so the production kernel runs), the
 7B-config lookahead shape W15 N5 G15 on the tiny model, and the edge shapes of tests/golden/greedy_edge_traces.json.gz
@@ -9,16 +11,19 @@ through the ENGINE (the state-machine replay of those traces is in test_gpu_stat
 Pass criterion: ids identical, or every divergence is a near-tie on the reference model's own logits (<= 3 bf16 ulps
 below its top logit for both candidates); every position is compared (the reference's token is forced after a
 divergence).  The report is printed (run with -s) and the exact cases are asserted exact."""
+import functools
+import gzip
+import json
+import os
 import random
 
 import pytest
 import torch
 
 from baseline import parity as PAR
-from baseline import ref_loader as R
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not R.reference_available(), reason="unmodified reference not present (baseline/_ref)")]
+pytestmark = pytest.mark.gpu
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_gpu_parity.json.gz")
 
 TINY = dict(hidden=256, layers=2, heads=2, kv_heads=2, inter=688, vocab=32000, max_pos=2048, rope_theta=10000.0, eps=1e-5)
 GQA = dict(hidden=512, layers=2, heads=4, kv_heads=2, inter=688, vocab=4096, max_pos=2048, rope_theta=10000.0, eps=1e-5)
@@ -44,14 +49,24 @@ CASES = [("cfg1_w5n3g3",       TINY, 5,  3, 3,  64, 96, False),
          ("edge_w2n4g1",       TINY, 2,  4, 1,  16, 32, True),
          ("edge_g1_w15n5",     TINY, 15, 5, 1,  32, 48, True),
          ("edge_n3_w20g20",    TINY, 20, 3, 20, 24, 48, True)]
+FP16_CASES = ("cfg1_w5n3g3_pool", "w15n5g15", "gqa_w15n5g15", "d64_gqa_w15n5g15", "edge_p1")
 
 
-def build_pair(shape, seed=0, dtype=torch.bfloat16):
+@functools.lru_cache(maxsize=None)
+def _records():
+    with gzip.open(GOLDEN, "rt") as f:
+        return json.load(f)["records"]
+
+
+def build_recorded(key, shape, dtype=torch.bfloat16):
+    """The HF model (bench.build_model, seed 0) and the record of the reference's run on those weights."""
     from bench import build_model
-    hf = build_model(shape, torch.device("cuda"), seed=seed)
+    hf = build_model(shape, torch.device("cuda"), seed=0)
     if dtype != torch.bfloat16:
         hf = hf.to(dtype)
-    return hf, PAR.reference_model_sharing_weights(hf, shape)
+    rec = _records()[key]
+    assert PAR.weights_digest(hf) == rec["weights_sha256"], f"{key}: not the weights the reference was recorded on"
+    return hf, rec
 
 
 def engine_generate(hf, W, N, G, pool, cap, eos=(), **engine_kw):
@@ -65,32 +80,26 @@ def engine_generate(hf, W, N, G, pool, cap, eos=(), **engine_kw):
 
 @pytest.mark.parametrize("name,shape,W,N,G,P,new,pool", CASES, ids=[c[0] for c in CASES])
 def test_engine_ids_match_reference_on_the_same_gpu(name, shape, W, N, G, P, new, pool):
-    hf, ref = build_pair(shape)
-    g = torch.Generator().manual_seed(1)
-    prompt = torch.randint(3, shape["vocab"], (P,), generator=g).tolist()
-    ref_ids, ref_steps = PAR.reference_greedy(ref, prompt, new, W, N, G, py_seed=0, pool_from_prompt=pool)
-    assert len(ref_ids) == P + new
+    hf, rec = build_recorded(name, shape)
+    assert len(rec["ids"]) == P + new and rec["n_prompt"] == P
     eng, gen = engine_generate(hf, W, N, G, pool, P + new)
-    rep = PAR.compare_ids(gen, ref_ids, P, ref)
+    rep = PAR.compare_ids_to_record(gen, rec, shape["vocab"])
     print(f"\n{name}: exact={rep['exact']} exact_prefix={rep['exact_prefix_tokens']}/{rep['compared_tokens']} "
           f"divergences={rep['n_divergences']} worst={rep['worst_candidate_below_top_ulps']} ulp "
-          f"ref_steps={ref_steps} {rep['divergences'][:3]}")
+          f"ref_steps={rec['steps']} {rep['divergences'][:3]}")
     assert rep["ok"], rep
     eng.close()
 
 
 def test_eos_on_first_token_matches_reference():
-    hf, ref = build_pair(TINY)
-    g = torch.Generator().manual_seed(1)
-    prompt = torch.randint(3, 32000, (12,), generator=g).tolist()
-    free, _ = PAR.reference_greedy(ref, prompt, 16, 5, 3, 3, py_seed=0, pool_from_prompt=True)
-    eos = free[12]
-    ref_ids, _ = PAR.reference_greedy(ref, prompt, 16, 5, 3, 3, py_seed=0, eos_token_id=[eos], pool_from_prompt=True)
-    assert ref_ids == prompt + [eos]
+    hf, rec = build_recorded("eos_first", TINY)
+    ref_ids = rec["ids"]
+    prompt, eos = ref_ids[:12], ref_ids[12]
+    assert len(ref_ids) == 12 + 1          # the reference stopped on the EOS it emitted first
     eng, gen = engine_generate(hf, 5, 3, 3, True, 12 + 16, eos=[eos])
     ours = gen(prompt, 16)
     if ours != ref_ids:      # only a near-tie on the very first token may differ
-        rep = PAR.compare_ids(gen, ref_ids, 12, ref)
+        rep = PAR.compare_ids_to_record(gen, rec, 32000)
         assert rep["ok"], rep
     eng.close()
 
@@ -100,15 +109,12 @@ def test_window_fill_step_larger_than_steady_and_host_stopping_criteria():
     silent clamp); output == the reference model's plain greedy.  Then a custom StoppingCriteria through generate()."""
     import lade
     from transformers import StoppingCriteria, StoppingCriteriaList
-    hf, ref = build_pair(TINY)
-    g = torch.Generator().manual_seed(3)
-    prompt = torch.randint(3, 32000, (10,), generator=g).tolist()
-    ar = list(prompt)
-    for _ in range(24):
-        ar.append(int(torch.argmax(PAR.reference_next_logits(ref, ar))))
+    hf, rec = build_recorded("plain_greedy", TINY)
+    prompt = rec["ids"][:10]
+    assert len(rec["ids"]) == 10 + 24
     eng, gen = engine_generate(hf, 5, 8, 0, False, 10 + 24)
     assert eng.q_nonprefill > eng.q_steady
-    rep = PAR.compare_ids(gen, ar, 10, ref)
+    rep = PAR.compare_ids_to_record(gen, rec, 32000)
     assert rep["ok"], rep
     eng.close()
 
@@ -135,22 +141,19 @@ def test_window_fill_step_larger_than_steady_and_host_stopping_criteria():
         os.environ["USE_LADE"] = "0"
 
 
-@pytest.mark.parametrize("name,shape,W,N,G,P,new,pool", [c for c in CASES if c[0] in ("cfg1_w5n3g3_pool", "w15n5g15", "gqa_w15n5g15",
-                                                                                     "d64_gqa_w15n5g15", "edge_p1")],
+@pytest.mark.parametrize("name,shape,W,N,G,P,new,pool", [c for c in CASES if c[0] in FP16_CASES],
                          ids=lambda v: v if isinstance(v, str) else None)
 def test_fp16_engine_ids_match_reference_on_the_same_gpu(name, shape, W, N, G, P, new, pool):
     """fp16 models (the dtype of the reference's README / minimal.py): the *_f16 kernels against the unmodified reference
     running in fp16 on the same GPU and weights; ties are measured in fp16 ulps."""
-    hf, ref = build_pair(shape, dtype=torch.float16)
-    assert next(ref.parameters()).dtype == torch.float16
-    g = torch.Generator().manual_seed(1)
-    prompt = torch.randint(3, shape["vocab"], (P,), generator=g).tolist()
-    ref_ids, ref_steps = PAR.reference_greedy(ref, prompt, new, W, N, G, py_seed=0, pool_from_prompt=pool)
+    hf, rec = build_recorded("fp16/" + name, shape, dtype=torch.float16)
+    assert rec["mant_bits"] == 10 and len(rec["ids"]) == P + new
+    prompt = rec["ids"][:P]
     eng, gen = engine_generate(hf, W, N, G, pool, P + new)
     assert eng.dt == torch.float16
-    rep = PAR.compare_ids(gen, ref_ids, P, ref)
+    rep = PAR.compare_ids_to_record(gen, rec, shape["vocab"])
     print(f"\nfp16 {name}: exact={rep['exact']} exact_prefix={rep['exact_prefix_tokens']}/{rep['compared_tokens']} "
-          f"divergences={rep['n_divergences']} worst={rep['worst_candidate_below_top_ulps']} ulp(fp16) ref_steps={ref_steps}")
+          f"divergences={rep['n_divergences']} worst={rep['worst_candidate_below_top_ulps']} ulp(fp16) ref_steps={rec['steps']}")
     assert rep["ok"], rep
     # sampling on the fp16 logits (device verification): reproducible, in range
     a = eng.generate(prompt, min(new, 24), rng=random.Random(1), sampling={"temperature": 0.8, "top_k": 40, "seed": 5})
@@ -163,12 +166,9 @@ def test_fp16_engine_ids_match_reference_on_the_same_gpu(name, shape, W, N, G, P
                          ids=["w15n5g15_pool", "w20n7g20_pool", "gqa_w15n5g15", "edge_p1"])
 def test_reference_order_attention_engine_ids(name, shape, W, N, G, P, new, pool):
     """attn_impl=3: the attention variant that rounds the probabilities like the reference, through the whole engine."""
-    hf, ref = build_pair(shape)
-    g = torch.Generator().manual_seed(1)
-    prompt = torch.randint(3, shape["vocab"], (P,), generator=g).tolist()
-    ref_ids, _ = PAR.reference_greedy(ref, prompt, new, W, N, G, py_seed=0, pool_from_prompt=pool)
+    hf, rec = build_recorded(name, shape)
     eng, gen = engine_generate(hf, W, N, G, pool, P + new, attn_impl=3)
-    rep = PAR.compare_ids(gen, ref_ids, P, ref)
+    rep = PAR.compare_ids_to_record(gen, rec, shape["vocab"])
     print(f"\n{name} (attn_impl=3): exact={rep['exact']} divergences={rep['n_divergences']}")
     assert rep["ok"], rep
     eng.close()

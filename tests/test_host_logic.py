@@ -151,9 +151,10 @@ def test_config_lade_joins_lookahead_workers_over_gloo(tmp_path):
         "dist.barrier()\n"
         "print('LP_JOIN_OK') if dist.get_rank() == 0 else None\n"
         "dist.destroy_process_group()\n")
+    # host only: with a GPU visible every worker selects the device of its LOCAL_RANK, which a one-GPU machine lacks
     res = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2",
                           "--master-addr", "127.0.0.1", "--master-port", "29581", str(script)],
-                         capture_output=True, text=True, timeout=300)
+                         capture_output=True, text=True, timeout=300, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
     assert res.returncode == 0 and "LP_JOIN_OK" in res.stdout, res.stderr[-1500:]
 
 
